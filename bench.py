@@ -8,6 +8,7 @@ error-bound sampler runs all 5 rounds — the worst case) through hold_render_fg
 feature, skinning Jacobian, colour net, density) -> n-way merge + volume integration, for every node.
 
   python bench.py --gpus N --steps K --warmup W            # ours (torchrun for N > 1)
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/<name>.npy
   python bench.py --impl reference [--steps K]             # the reference algorithm on the host CPU cores
 
 Rays shard over ranks with no data-path collective (render.py has no gradients, SURVEY D4): each rank renders
@@ -315,10 +316,32 @@ def run_train(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out, path):
+    """Every tensor of one forward_fg result as <path>/<key>.npy: floating outputs as float32, integer ones as float64 (exact).
+    The benchmark's workload gives 48 floats per ray, 50.3 MB for the 512x512 frame."""
+    import numpy as np
+
+    arrays = {k: v.detach().cpu() for k, v in out.items() if torch.is_tensor(v)}
+    arrays = {k: (v.float() if v.is_floating_point() else v.double()).numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    # H, W and NODES are constants, so the whole result always fits; a larger frame would need a fixed, seeded sample of rays
+    assert total <= 64e6, f"outputs of {total / 1e6:.1f} MB exceed the 64 MB a dump may hold"
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=positive_int, default=3, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default=os.environ.get("HOLD_MLP_MODE", "auto"), choices=["auto", "fp32", "tc"])
@@ -327,7 +350,12 @@ def main():
     ap.add_argument("--config", default="render", choices=["render", "train"],
                     help="render: BASELINE configs[1] (the driver's line); train: one data-parallel training step (configs[4] / SURVEY C5)")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2] (two hands + object) and full-forward (with background) fields")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (rank 0); the inputs are "
+                         "seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != "render"):
+        ap.error("--dump-outputs applies to --impl ours --config render")
     if args.impl == "reference":
         return run_reference(args)
     if args.config == "train":
@@ -513,6 +541,8 @@ def main():
         "env": {k: v for k, v in os.environ.items() if k.startswith("HOLD_")},   # the library reads no environment; these steer bench.py only
     }
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(o, args.dump_outputs)
     if dist is not None:
         dist.destroy_process_group()
 

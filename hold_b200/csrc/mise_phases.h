@@ -7,7 +7,7 @@
 //              adding the 27 lattice points of the finer level                                  (mise.pyx:96-111,183-273)
 //   to_dense(): known values on the (R+1)^3 lattice, NaN elsewhere, forward-filled along x, then y, then z (:138-166)
 // The per-item functions below compile for the host too (tests/host/mise_host.cpp), where they are checked against the
-// reference's own compiled MISE (oracle/_ref, built by oracle/build_ref_mise.py).
+// oracle's restatement of mise.pyx (oracle/mise_oracle.py, pinned to a recorded run of the reference's compiled MISE).
 #pragma once
 #include <math.h>
 #include <stdint.h>

@@ -1,14 +1,15 @@
-"""CPU-only, SURVEY §8f rank 4: the MISE restatement the CUDA kernels run (hold_b200/csrc/mise_phases.h, compiled for the
-host) against the REFERENCE's own compiled Cython MISE (oracle/_ref/mise*.so from oracle/build_ref_mise.py; the built module
-travels with the repo snapshot, /root/reference is only needed to build it) — round by round and bit for bit."""
+"""CPU-only, SURVEY §8f rank 4.  The oracle's restatement of the reference's Cython MISE (oracle/mise_oracle.py, the reference's
+own octree) is pinned to a run of the reference's compiled module recorded in profiles/r02_bench_aux.jsonl; the MISE
+restatement the CUDA kernels run (hold_b200/csrc/mise_phases.h, compiled for the host) is held to the oracle round by round
+and bit for bit."""
 import ctypes as C
-import glob
 import os
 import subprocess
-import sys
 
 import numpy as np
 import pytest
+
+from oracle import mise_oracle
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -30,19 +31,6 @@ def _host():
     return lib
 
 
-def _ref_mise():
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import build_ref_mise
-
-    so = build_ref_mise.build() or next(iter(glob.glob(os.path.join(ROOT, "oracle", "_ref", "mise*.so"))), None)
-    if so is None:
-        pytest.skip("reference MISE not built (needs /root/reference once)")
-    sys.path.insert(0, os.path.dirname(so))
-    import mise
-
-    return mise
-
-
 def _field(seed):
     rng = np.random.default_rng(seed)
     c = rng.uniform(0.3, 0.7, size=(3, 3))
@@ -57,10 +45,10 @@ def _field(seed):
 
 
 @pytest.mark.parametrize("res0,depth,seed", [(4, 2, 0), (4, 3, 1), (8, 2, 2), (6, 3, 3), (32, 2, 4)])
-def test_mise_restatement_matches_reference_mise(res0, depth, seed):
-    lib, mise = _host(), _ref_mise()
+def test_host_mise_matches_mise_oracle(res0, depth, seed):
+    lib = _host()
     f = _field(seed)
-    ref = mise.MISE(res0, depth, 0.0)
+    ref = mise_oracle.MISE(res0, depth, 0.0)
     h = lib.mise_host_create(res0, depth, C.c_float(0.0))
     R = res0 << depth
     G = R + 1
@@ -85,3 +73,31 @@ def test_mise_restatement_matches_reference_mise(res0, depth, seed):
     lib.mise_host_to_dense(h, out.ctypes.data_as(C.c_void_p))
     lib.mise_host_destroy(h)
     assert np.array_equal(out.reshape(G, G, G).astype(np.float64), dense_ref)
+
+
+def test_mise_oracle_reproduces_recorded_reference_run():
+    """tools/bench_aux.py row 8f-4a drove the reference's compiled MISE (32 -> 256, threshold 0) with the oracle's SDF net on the
+    canonical object of synth.make_scene(H=8, W=8, S=32, seed=4), through the point mapping of utils/meshing.py:24-32, and
+    recorded 845 872 SDF queries (profiles/r02_bench_aux.jsonl).  The oracle replays that run: which voxels subdivide in which
+    round decides every count, so an error in the marking or subdivision rules moves it."""
+    import torch
+    from hold_b200 import synth
+    from oracle import hold_oracle as O
+
+    torch.set_num_threads(min(8, os.cpu_count() or 1))
+    sc = synth.make_scene(H=8, W=8, S=32, nodes=("right", "object"), seed=4)
+    v = sc.obj_pts_cano.numpy().astype(np.float32)
+    center, scale = (v.min(0) + v.max(0)) * 0.5, (v.max(0) - v.min(0)).max()
+    ex = mise_oracle.MISE(32, 3, 0.0)
+    per_round = []
+    pts = ex.query()
+    with torch.no_grad():
+        while pts.shape[0] != 0:
+            p = (pts.astype(np.float32) / ex.resolution - 0.5) * 1.1
+            p = p * scale + center
+            vals = O.sdf_mlp(torch.tensor(p).float(), sc.sdf_state["object"])[:, 0].numpy().astype(np.float64)
+            per_round.append(pts.shape[0])
+            ex.update(pts, vals)
+            pts = ex.query()
+    print("queries per round", per_round)
+    assert sum(per_round) == 845872

@@ -1,26 +1,17 @@
-"""SURVEY §8f rank 4: the GPU MISE + fused-MLP SDF queries against the reference's own compiled MISE (oracle/_ref, travels
-with the snapshot) fed with the SAME SDF values round by round -> identical dense grids.  The restatement itself is already
-checked bit for bit on the CPU (tests/test_cpu_mise.py); green on hardware since round 1, strict since round 2."""
-import glob
-import os
-import sys
-
+"""SURVEY §8f rank 4: the GPU MISE + fused-MLP SDF queries against the oracle's restatement of the reference's MISE
+(oracle/mise_oracle.py, the reference's own octree) fed with the SAME SDF values round by round -> identical dense grids.  The
+oracle's pin to a recorded run of the reference's compiled MISE, and the kernels' restatement against the oracle on the host,
+are in tests/test_cpu_mise.py."""
 import numpy as np
 import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def impl_generate_grid_matches_reference_mise(ctx):
+def impl_generate_grid_matches_mise_oracle(ctx):
     from hold_b200 import capi, meshing, scene_io, synth
-
-    so = next(iter(glob.glob(os.path.join(ROOT, "oracle", "_ref", "mise*.so"))), None)
-    if so is None:
-        pytest.skip("reference MISE not built")
-    sys.path.insert(0, os.path.dirname(so))
-    import mise
+    from oracle import mise_oracle
 
     dev = torch.device("cuda", 0)
     sc = synth.make_scene(H=8, W=8, S=32, nodes=("right", "object"), seed=4)
@@ -30,8 +21,8 @@ def impl_generate_grid_matches_reference_mise(ctx):
     verts = sc.obj_pts_cano.numpy()
     grid, res, gt_scale, gt_center = meshing.generate_grid(ctx, func, verts, 0.0, res_init=8, res_up=2)
     ctx.check()
-    # the reference loop (utils/meshing.py:19-47) with the same SDF function
-    ex = mise.MISE(8, 2, 0.0)
+    # the reference's loop (utils/meshing.py:19-47) with the same SDF function
+    ex = mise_oracle.MISE(8, 2, 0.0)
     pts = ex.query()
     rounds = 0
     while pts.shape[0] != 0:
@@ -48,5 +39,5 @@ def impl_generate_grid_matches_reference_mise(ctx):
     assert (grid < 0).any() and (grid > 0).any()
 
 
-def test_generate_grid_matches_reference_mise(isolated):
-    isolated("tests/test_gpu_mise.py", "impl_generate_grid_matches_reference_mise")
+def test_generate_grid_matches_mise_oracle(isolated):
+    isolated("tests/test_gpu_mise.py", "impl_generate_grid_matches_mise_oracle")
