@@ -101,6 +101,12 @@ EXPORTS = {
     "hold_rgb_eval": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, fp, fp, fp, fp, fp, fp, C.c_void_p]),
     "hold_forward_warp": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, fp, C.POINTER(NodePose), fp, fp, fp, C.c_void_p]),
     "hold_inverse_warp": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, fp, C.POINTER(NodePose), fp, fp, fp, C.c_void_p]),
+    "hold_train_glue_sizes": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "hold_normal_density": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int] + [fp] * 8 + [C.c_void_p]),
+    "hold_normal_density_bwd": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int] + [fp] * 11 + [C.c_void_p]),
+    "hold_bg_inputs": (C.c_int, [C.c_void_p, C.c_int, C.c_float, fp, fp, fp, fp, C.c_void_p]),
+    "hold_bg_integrate": (C.c_int, [C.c_void_p, C.c_int, C.c_float, fp, C.c_int, fp, fp, fp, fp, fp, C.c_void_p]),
+    "hold_bg_integrate_bwd": (C.c_int, [C.c_void_p, C.c_int, C.c_float, fp, C.c_int, fp, fp, fp, fp, fp, fp, fp, fp, C.c_void_p]),
 }
 
 _lib = None

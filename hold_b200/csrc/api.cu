@@ -20,6 +20,7 @@
 #include "warp_bwd.cuh"
 #include "train.cuh"
 #include "wgrad_tc.cuh"
+#include "train_glue.cuh"
 
 namespace hold {
 
@@ -1241,6 +1242,106 @@ int hold_inverse_warp(hold_ctx* ctx, int node, int B, int P, const float* x, con
   HOLD_REQUIRE(x && pose && x_c && pose->tfs, "NULL argument");
   return launch_inverse_warp(ctx, ctx->nodes[node], B, P, false, 1, 1, nullptr, nullptr, nullptr, x, pose, x_c, knn_idx,
                              outlier_mask, nullptr, (cudaStream_t)stream);
+}
+
+// ------------------------------------------------------------------------------------------------ training glue (train_glue.cuh)
+static int nd_blocks(int P) { return max(1, ceil_div(P, kGlueThreads)); }
+
+int hold_train_glue_sizes(hold_ctx* ctx, int node, int B, int P, int64_t* stash_floats, int64_t* scratch_floats) {
+  int rc = check_node(ctx, node, false);
+  if (rc) return rc;
+  HOLD_REQUIRE(B >= 0 && P >= 0, "negative size");
+  const bool hand = ctx->nodes[node].cfg.kind == HOLD_KIND_HAND;
+  if (stash_floats) *stash_floats = (int64_t)B * P * (hand ? glue::kStashHand : glue::kStashObj);
+  if (scratch_floats) *scratch_floats = (int64_t)B * nd_blocks(P) * (hand ? glue::kPartHand : glue::kPartObj);
+  return HOLD_OK;
+}
+
+int hold_normal_density(hold_ctx* ctx, int node, int B, int P, const float* x_c, const float* grad, const float* sdf,
+                        const float* tfs, const float* beta, float* normal, float* density, float* stash, void* stream) {
+  int rc = check_node(ctx, node, false);
+  if (rc) return rc;
+  HOLD_REQUIRE(B >= 0 && P >= 0, "negative size");
+  if (B * P == 0) return HOLD_OK;
+  HOLD_REQUIRE(grad && sdf && tfs && beta && normal && density && stash, "NULL argument");
+  NodeState& ns = ctx->nodes[node];
+  const bool hand = ns.cfg.kind == HOLD_KIND_HAND;
+  dim3 grid(nd_blocks(P), B);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (hand) {
+    HOLD_REQUIRE(ns.has_rig, "hand node has no rig (hold_node_set_rig)");
+    HOLD_REQUIRE(x_c != nullptr, "hand node needs x_c for the skinning weights");
+    k_nd_fwd<true><<<grid, kGlueThreads, 0, s>>>(P, x_c, grad, sdf, tfs, ns.cano_verts, ns.skin_w, beta, normal, density, stash);
+  } else {
+    k_nd_fwd<false><<<grid, kGlueThreads, 0, s>>>(P, x_c, grad, sdf, tfs, nullptr, nullptr, beta, normal, density, stash);
+  }
+  HOLD_LAUNCH_CHECK(ctx);
+  return HOLD_OK;
+}
+
+int hold_normal_density_bwd(hold_ctx* ctx, int node, int B, int P, const float* grad, const float* sdf, const float* beta,
+                            const float* stash, const float* d_normal, const float* d_density, float* d_grad, float* d_sdf,
+                            float* d_tfs, float* d_beta, float* scratch, void* stream) {
+  int rc = check_node(ctx, node, false);
+  if (rc) return rc;
+  HOLD_REQUIRE(B >= 0 && P >= 0, "negative size");
+  if (B == 0) return HOLD_OK;
+  HOLD_REQUIRE(beta && d_tfs && d_beta && scratch, "NULL argument");
+  HOLD_REQUIRE(P == 0 || (grad && sdf && stash && d_grad && d_sdf), "NULL argument");
+  const bool hand = ctx->nodes[node].cfg.kind == HOLD_KIND_HAND;
+  const int nb = nd_blocks(P);
+  dim3 grid(nb, B);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (hand) {
+    k_nd_bwd<true><<<grid, kGlueThreads, 0, s>>>(P, grad, sdf, beta, stash, d_normal, d_density, d_grad, d_sdf, scratch);
+    HOLD_LAUNCH_CHECK(ctx);
+    k_nd_bwd_final<true><<<B, 256, 0, s>>>(nb, scratch, d_tfs, d_beta);
+  } else {
+    k_nd_bwd<false><<<grid, kGlueThreads, 0, s>>>(P, grad, sdf, beta, stash, d_normal, d_density, d_grad, d_sdf, scratch);
+    HOLD_LAUNCH_CHECK(ctx);
+    k_nd_bwd_final<false><<<B, 16, 0, s>>>(nb, scratch, d_tfs, d_beta);
+  }
+  HOLD_LAUNCH_CHECK(ctx);
+  return HOLD_OK;
+}
+
+int hold_bg_inputs(hold_ctx* ctx, int R, float r_sphere, const float* cam_loc, const float* ray_dirs, float* emb_pts,
+                   float* emb_view, void* stream) {
+  HOLD_REQUIRE(ctx != nullptr, "ctx is NULL");
+  HOLD_REQUIRE(R >= 0 && r_sphere > 0.f, "bad R / r_sphere");
+  if (R == 0) return HOLD_OK;
+  HOLD_REQUIRE(cam_loc && ray_dirs && emb_pts && emb_view, "NULL argument");
+  HOLD_CUDA(cudaSetDevice(ctx->device));
+  k_bg_inputs<<<ceil_div(R * kBgN, kGlueThreads), kGlueThreads, 0, (cudaStream_t)stream>>>(R, r_sphere, cam_loc, ray_dirs, emb_pts, emb_view);
+  HOLD_LAUNCH_CHECK(ctx);
+  return HOLD_OK;
+}
+
+int hold_bg_integrate(hold_ctx* ctx, int R, float r_sphere, const float* sdf, int ld_sdf, const float* rgb, const float* fg_bg_weights,
+                      float* bg_rgb, float* bg_rgb_only, float* bg_semantics, void* stream) {
+  HOLD_REQUIRE(ctx != nullptr, "ctx is NULL");
+  HOLD_REQUIRE(R >= 0 && r_sphere > 0.f && ld_sdf >= 1, "bad R / r_sphere / ld_sdf");
+  if (R == 0) return HOLD_OK;
+  HOLD_REQUIRE(sdf && rgb && fg_bg_weights, "NULL argument");
+  HOLD_CUDA(cudaSetDevice(ctx->device));
+  k_bg_integrate<<<ceil_div(R, kGlueThreads), kGlueThreads, 0, (cudaStream_t)stream>>>(R, r_sphere, sdf, ld_sdf, rgb, fg_bg_weights, bg_rgb,
+                                                                                    bg_rgb_only, bg_semantics);
+  HOLD_LAUNCH_CHECK(ctx);
+  return HOLD_OK;
+}
+
+int hold_bg_integrate_bwd(hold_ctx* ctx, int R, float r_sphere, const float* sdf, int ld_sdf, const float* rgb,
+                          const float* fg_bg_weights, const float* g_bg_rgb, const float* g_bg_rgb_only, const float* g_bg_semantics,
+                          float* d_rgb, float* d_sdf, float* d_fg_bg_weights, void* stream) {
+  HOLD_REQUIRE(ctx != nullptr, "ctx is NULL");
+  HOLD_REQUIRE(R >= 0 && r_sphere > 0.f && ld_sdf >= 1, "bad R / r_sphere / ld_sdf");
+  if (R == 0) return HOLD_OK;
+  HOLD_REQUIRE(sdf && rgb && fg_bg_weights && d_rgb && d_sdf && d_fg_bg_weights, "NULL argument");
+  HOLD_CUDA(cudaSetDevice(ctx->device));
+  k_bg_integrate_bwd<<<ceil_div(R, kGlueThreads), kGlueThreads, 0, (cudaStream_t)stream>>>(R, r_sphere, sdf, ld_sdf, rgb, fg_bg_weights, g_bg_rgb,
+                                                                                        g_bg_rgb_only, g_bg_semantics, d_rgb, d_sdf, d_fg_bg_weights);
+  HOLD_LAUNCH_CHECK(ctx);
+  return HOLD_OK;
 }
 
 }  // extern "C"

@@ -13,9 +13,10 @@ The second-order path of the reference (normals feed the colour net with create_
 d sdf / d x_c is an OUTPUT of SdfNetFn and its backward takes a seed for it (train_algo.sdf_backward).
 
 What stays in PyTorch on purpose (host code per BASELINE.json north_star: "Host code stays Python/PyTorch for the training loop"):
-weight-norm folding of the parameters, losses, the optimiser; and, in this first version, the per-point 3x3 normal algebra, the
-Laplace density and the n-way merge + volume integration of the 1 280-ray training batch (tiny next to the nets; their fused
-inference kernels exist, their backward twins are the next step: DESIGN.md)."""
+weight-norm folding of the parameters, losses, the optimiser; and, by default, the per-point 3x3 normal algebra, the Laplace
+density and the background's inputs and 32-sample integration.  fused=True (node_forward_train, background_forward_train,
+forward_train, TrainStep) runs that glue on hold_normal_density / hold_bg_inputs / hold_bg_integrate and their backward twins
+(NormalDensityFn, BgIntegrateFn; hold_b200/csrc/train_glue.cuh) instead."""
 from __future__ import annotations
 
 import ctypes as C
@@ -294,18 +295,67 @@ def laplace_density(sdf, beta):
     return (1.0 / beta) * (0.5 + 0.5 * sdf.sign() * torch.expm1(-sdf.abs() / beta))
 
 
-def node_forward_train(node, x, tfs, verts, frame_of_point, pose_cond=None, time_code=None, sync=True):
+def _glue_sizes(node, B, P):
+    """floats of hold_normal_density's stash and of hold_normal_density_bwd's scratch for B x P points of the node"""
+    st, sc = C.c_int64(), C.c_int64()
+    check(lib().hold_train_glue_sizes(node.ctx.h, node.slot, B, P, C.byref(st), C.byref(sc)))
+    return st.value, sc.value
+
+
+class NormalDensityFn(torch.autograd.Function):
+    """(normal [B*P,3], density [B*P]) of a node's frame-major samples in one kernel (hold_normal_density): the normal of
+    extract_features (volsdf_utils.py:66-102) = normalize(g . J^-1) with J the forward-skinning Jacobian under detached weights, and
+    the Laplace density (density.py:21-26) at the effective beta.  Differentiable w.r.t. g, sdf, tfs and beta; x_c only selects
+    the hand's skinning weights (detached in the reference, deformer.py:101).  The backward (hold_normal_density_bwd) reads the
+    forward's per-point stash (J^-1 and the blended weights), so the KNN runs once."""
+
+    @staticmethod
+    def forward(fctx, node, B, x_c, g, sdf, tfs, beta):
+        fctx.set_materialize_grads(False)
+        P = x_c.shape[0] // B
+        dev = g.device
+        f = lambda t: t.detach().float().contiguous()
+        xc, gg, s, tf, bt = f(x_c), f(g), f(sdf), f(tfs), f(beta).reshape(1)
+        n_stash, _ = _glue_sizes(node, B, P)
+        normal, density = torch.empty(B * P, 3, device=dev), torch.empty(B * P, device=dev)
+        stash = torch.empty(n_stash, device=dev)
+        check(lib().hold_normal_density(node.ctx.h, node.slot, B, P, ptr(xc), ptr(gg), ptr(s), ptr(tf), ptr(bt), ptr(normal),
+                                        ptr(density), ptr(stash), stream_ptr()))
+        fctx.node, fctx.B, fctx.P, fctx.keep = node, B, P, (gg, s, bt, stash)
+        fctx.tfs_shape, fctx.beta_shape = tfs.shape, beta.shape
+        return normal, density
+
+    @staticmethod
+    def backward(fctx, d_normal, d_density):
+        node, B, P = fctx.node, fctx.B, fctx.P
+        gg, s, bt, stash = fctx.keep
+        dev = gg.device
+        f = lambda t: None if t is None else t.float().contiguous()
+        dn, dd = f(d_normal), f(d_density)
+        _, n_scratch = _glue_sizes(node, B, P)
+        d_g, d_s = torch.empty_like(gg), torch.empty_like(s)
+        d_tfs, d_beta = torch.empty(fctx.tfs_shape, device=dev), torch.empty(1, device=dev)
+        scratch = torch.empty(n_scratch, device=dev)
+        check(lib().hold_normal_density_bwd(node.ctx.h, node.slot, B, P, ptr(gg), ptr(s), ptr(bt), ptr(stash), ptr(dn), ptr(dd),
+                                            ptr(d_g), ptr(d_s), ptr(d_tfs), ptr(d_beta), ptr(scratch), stream_ptr()))
+        return None, None, None, d_g, d_s, d_tfs, d_beta.reshape(fctx.beta_shape)
+
+
+def node_forward_train(node, x, tfs, verts, frame_of_point, pose_cond=None, time_code=None, sync=True, fused=False):
     """Node.forward after sampling, training mode (node.py:57-87 + volsdf_utils.py:51-147): deformed points x [B,P,3] ->
     dict(sdf, x_c, feat, grad, normal, color, density), everything differentiable w.r.t. the node's parameters, tfs, beta,
-    the frame / pose codes.  `verts`: posed vertices (hand).  frame_of_point [B*P] long."""
+    the frame / pose codes.  `verts`: posed vertices (hand).  frame_of_point [B*P] long.
+    fused: normal and density from one kernel and its backward twin (NormalDensityFn) instead of the torch ops below."""
     if sync:
         node.sync_weights()
     B, P, _ = x.shape
     x_c = InverseWarpFn.apply(node, x, tfs, verts).reshape(B * P, 3)
     Ws, bs = _folded_sdf(node)
     sdf, feat, g = SdfNetFn.apply(node, x_c, *Ws, *bs)
+    if fused:
+        normal, density = NormalDensityFn.apply(node, B, x_c, g, sdf, tfs, node.density.get_beta())
     # J of forward skinning with detached weights (volsdf_utils.py:66-81): sum_j w_j tfs_j[:3,:3]; hand: KNN vs canonical verts
-    if node.kind == "hand":
+    elif node.kind == "hand":
         pose = NodePose()
         tf = tfs.detach().float().contiguous()
         pose.tfs = tf.data_ptr()
@@ -322,8 +372,9 @@ def node_forward_train(node, x, tfs, verts, frame_of_point, pose_cond=None, time
         J = torch.bmm(w.reshape(B, P, 16), tfs[:, :, :3, :3].reshape(B, 16, 9)).reshape(B * P, 3, 3)
     else:
         J = tfs.reshape(B, 1, 4, 4)[:, :, :3, :3].expand(B, P, 3, 3).reshape(B * P, 3, 3)
-    # inv_ex: torch.linalg.inv reads its error flag on the host (a sync per node per step)
-    normal = torch.nn.functional.normalize(torch.einsum("bi,bij->bj", g, torch.linalg.inv_ex(J).inverse), dim=1, eps=1e-6)
+    if not fused:
+        # inv_ex: torch.linalg.inv reads its error flag on the host (a sync per node per step)
+        normal = torch.nn.functional.normalize(torch.einsum("bi,bij->bj", g, torch.linalg.inv_ex(J).inverse), dim=1, eps=1e-6)
     if node.kind == "hand":
         pe = node.rendering_network.lin_pose(pose_cond)[:, None, :].expand(B, P, 8).reshape(B * P, 8)   # per-frame rows, frame-major points
         inp = torch.cat([x_c, normal, pe, feat], 1)
@@ -331,7 +382,8 @@ def node_forward_train(node, x, tfs, verts, frame_of_point, pose_cond=None, time
         inp = torch.cat([x_c, normal, x_c.new_zeros(B * P, 8), feat, time_code[:, None, :].expand(B, P, 32).reshape(B * P, 32)], 1)
     Wr, br = _folded_rgb(node)
     color = RgbNetFn.apply(node, inp, *Wr, *br)
-    density = laplace_density(sdf, node.density.get_beta())
+    if not fused:
+        density = laplace_density(sdf, node.density.get_beta())
     return dict(sdf=sdf, x_c=x_c, feat=feat, grad=g, normal=normal, color=color, density=density)
 
 
@@ -470,25 +522,76 @@ def depth2pts_outside(ray_o, ray_d, depth, R_s):
     return torch.cat([pn, depth[..., None]], -1)
 
 
-def background_forward_train(bg, fg_bg_weights, ray_dirs, cam_loc, idx, B, R_s, n_bg=32, sync=True):
+class BgIntegrateFn(torch.autograd.Function):
+    """(bg_rgb [R,3], bg_rgb_only [R,3], bg_semantics [R,4]) = bg_volume_rendering of the 32 inverse-sphere samples per ray
+    (background.py:137-165, AbsDensity) + Background.forward's outputs (:35-54), on hold_bg_integrate / hold_bg_integrate_bwd.
+    sdf [R*32] may be a strided column (column 0 of BgSdfFn's output): the kernels take its stride, no copy.  Differentiable
+    w.r.t. sdf, rgb [R*32,3] and the foreground's bg_weights [R]."""
+
+    @staticmethod
+    def forward(fctx, ctx, R_s, sdf, rgb, fg_bg_weights):
+        fctx.set_materialize_grads(False)
+        assert sdf.dim() == 1 and sdf.dtype == torch.float32
+        R = fg_bg_weights.shape[0]
+        dev = rgb.device
+        s, c, w = sdf.detach(), rgb.detach().float().contiguous(), fg_bg_weights.detach().float().contiguous()
+        bg_rgb, only, sem = torch.empty(R, 3, device=dev), torch.empty(R, 3, device=dev), torch.empty(R, 4, device=dev)
+        check(lib().hold_bg_integrate(ctx.h, R, float(R_s), C.c_void_p(s.data_ptr()), s.stride(0), ptr(c), ptr(w), ptr(bg_rgb), ptr(only),
+                                      ptr(sem), stream_ptr()))
+        fctx.ctx, fctx.R_s, fctx.keep = ctx, float(R_s), (s, c, w)
+        return bg_rgb, only, sem
+
+    @staticmethod
+    def backward(fctx, g_rgb, g_only, g_sem):
+        s, c, w = fctx.keep
+        R = w.shape[0]
+        f = lambda t: None if t is None else t.float().contiguous()
+        d_rgb, d_sdf, d_w = torch.empty_like(c), torch.empty(s.shape[0], device=c.device), torch.empty_like(w)
+        check(lib().hold_bg_integrate_bwd(fctx.ctx.h, R, fctx.R_s, C.c_void_p(s.data_ptr()), s.stride(0), ptr(c), ptr(w), ptr(f(g_rgb)),
+                                          ptr(f(g_only)), ptr(f(g_sem)), ptr(d_rgb), ptr(d_sdf), ptr(d_w), stream_ptr()))
+        return None, None, d_sdf, d_rgb, d_w
+
+
+def bg_inputs(ctx, ray_dirs, cam_loc, R_s):
+    """The background nets' per-sample inputs without gradient (no parameter reaches them), one kernel (hold_bg_inputs):
+    -> PE-10 of depth2pts_outside at the 32 inverse-sphere depths [R*32, 84], PE-4 of the ray directions [R*32, 27]."""
+    R = ray_dirs.shape[0]
+    dev = ray_dirs.device
+    emb_pts, emb_view = torch.empty(R * 32, 84, device=dev), torch.empty(R * 32, 27, device=dev)
+    check(lib().hold_bg_inputs(ctx.h, R, float(R_s), ptr(cam_loc.detach().float().contiguous()), ptr(ray_dirs.detach().float().contiguous()),
+                               ptr(emb_pts), ptr(emb_view), stream_ptr()))
+    return emb_pts, emb_view
+
+
+def background_forward_train(bg, fg_bg_weights, ray_dirs, cam_loc, idx, B, R_s, n_bg=32, sync=True, fused=False):
     """Background.forward in training (background.py:35-100): -> dict(bg_rgb = bg_weights * bg_rgb_only, bg_rgb_only, bg_semantics),
     differentiable w.r.t. the background nets, its frame codes and the foreground's bg_weights.  Eval-mode (deterministic) inverse
-    sphere samples; the nets run on hold_linear (node -1), their weights must have been packed in tensor-core mode."""
+    sphere samples; the nets run on hold_linear (node -1), their weights must have been packed in tensor-core mode.
+    fused: the nets' inputs from one kernel (bg_inputs) and the 32-sample integration with its backward twin (BgIntegrateFn)
+    instead of the torch ops below."""
     if sync:
         bg.sync_weights()
     R = ray_dirs.shape[0]
     dev = ray_dirs.device
-    z = torch.flip(torch.linspace(0.0, 1.0, n_bg, device=dev) * (1.0 / R_s), dims=[-1])[None].expand(R, n_bg)       # 1/R_s ... 0
-    pts = depth2pts_outside(cam_loc[:, None, :].expand(R, n_bg, 3), ray_dirs[:, None, :].expand(R, n_bg, 3), z, R_s).reshape(R * n_bg, 4)
     fc = bg.frame_latent_encoder(idx)                                                                                  # [B,32]
     fcp = fc[:, None, :].expand(B, (R // B) * n_bg, 32).reshape(R * n_bg, 32)
-    inp = torch.cat([_embed_n(pts, 10), fcp], 1)
     Ws = [getattr(bg.bg_implicit_network, f"lin{l}").weight for l in range(9)]
     bs = [getattr(bg.bg_implicit_network, f"lin{l}").bias for l in range(9)]
+    rn = bg.bg_rendering_network
+    if fused:
+        assert n_bg == 32, "the fused background kernels take the reference's 32 samples"
+        emb_pts, view = bg_inputs(bg.ctx, ray_dirs, cam_loc, R_s)
+        out = BgSdfFn.apply(bg.ctx, torch.cat([emb_pts, fcp], 1), *Ws, *bs)
+        sdf, feat = out[:, 0], out[:, 1:]
+        rgb = BgRgbFn.apply(bg.ctx, torch.cat([view, fcp, feat], 1), rn.lin0.weight, rn.lin1.weight, rn.lin0.bias, rn.lin1.bias)
+        bg_rgb, only, sem = BgIntegrateFn.apply(bg.ctx, R_s, sdf, rgb, fg_bg_weights)
+        return dict(bg_rgb=bg_rgb, bg_rgb_only=only, bg_semantics=sem)
+    z = torch.flip(torch.linspace(0.0, 1.0, n_bg, device=dev) * (1.0 / R_s), dims=[-1])[None].expand(R, n_bg)       # 1/R_s ... 0
+    pts = depth2pts_outside(cam_loc[:, None, :].expand(R, n_bg, 3), ray_dirs[:, None, :].expand(R, n_bg, 3), z, R_s).reshape(R * n_bg, 4)
+    inp = torch.cat([_embed_n(pts, 10), fcp], 1)
     out = BgSdfFn.apply(bg.ctx, inp, *Ws, *bs)
     sdf, feat = out[:, 0], out[:, 1:]
     view = _embed_n(ray_dirs[:, None, :].expand(R, n_bg, 3).reshape(R * n_bg, 3), 4)
-    rn = bg.bg_rendering_network
     rgb = BgRgbFn.apply(bg.ctx, torch.cat([view, fcp, feat], 1), rn.lin0.weight, rn.lin1.weight, rn.lin0.bias, rn.lin1.bias).reshape(R, n_bg, 3)
     dens = sdf.abs().reshape(R, n_bg)                                                                                  # AbsDensity (density.py:33-35)
     dists = torch.cat([z[:, :-1] - z[:, 1:], torch.full((R, 1), 1e10, device=dev)], -1)
@@ -644,13 +747,14 @@ def prepare_loss_targets(out, node, B, P, canonical_pts, generator=None):
         out[f"{nid}.grad_theta"] = compute_gradient_samples(PointInSpace(global_sigma_xyz=xyz.cpu()), node, 256, v, B, 0.03, 0.20, generator)
 
 
-def forward_train(net, input, generator=None):
+def forward_train(net, input, generator=None, fused=False):
     """HOLDNet.forward in training mode (hold/hold_net.py:53-134) -> the reference's output dict: epoch, step, fg_rgb, fg_weights-free
     composite keys (mask_prob, normal, depth, fg_semantics, bg_weights), <node>.* of every node's own volumetric_render, the loss
     targets of prepare_loss_targets, bg_z_vals, ray_dirs, cam_loc, index, and (forward) rgb, semantics, bg_rgb_only.
     Every floating-point output carries the autograd graph to the nets, beta, poses / transforms and codes.  Training-mode rules
     mirrored: pose conditioning is zeroed while current_epoch < 20 (mano_node.py:82-85); sampling runs without gradients
-    (ray_sampler.py, torch.no_grad)."""
+    (ray_sampler.py, torch.no_grad).  fused: the per-point glue of the nodes and of the background on the fused kernels
+    (NormalDensityFn, bg_inputs, BgIntegrateFn)."""
     from . import ops
     from .model import ErrorBoundSampler
 
@@ -678,7 +782,7 @@ def forward_train(net, input, generator=None):
             if early:
                 pc = pc * 0.0
         o = node_forward_train(node, x, srv["tfs"] if hand else tfs, srv["verts"] if hand else None, fr.repeat_interleave(S),
-                               pose_cond=pc, time_code=None if hand else node.frame_latent_encoder(input["idx"]), sync=False)
+                               pose_cond=pc, time_code=None if hand else node.frame_latent_encoder(input["idx"]), sync=False, fused=fused)
         f = dict(color=o["color"].reshape(B * P, S, 3), normal=o["normal"].reshape(B * P, S, 3), density=o["density"].reshape(B * P, S), z_vals=z)
         factors.append(f)
         prepare_loss_targets(out, node, B, P, o["x_c"], generator)
@@ -692,7 +796,7 @@ def forward_train(net, input, generator=None):
     out["ray_dirs"], out["cam_loc"], out["index"] = dirs, cam, input["idx"]
     rgb, sem = comp["fg_rgb"], comp["fg_semantics"]
     if getattr(net, "background", None) is not None:                        # hold_net.py:110-134
-        bgo = background_forward_train(net.background, comp["bg_weights"], dirs, cam, input["idx"], B, R_s)
+        bgo = background_forward_train(net.background, comp["bg_weights"], dirs, cam, input["idx"], B, R_s, fused=fused)
         rgb, sem = rgb + bgo["bg_rgb"], sem + bgo["bg_semantics"]
         out["bg_rgb_only"] = bgo["bg_rgb_only"]
     out["rgb"], out["semantics"] = rgb, sem
@@ -762,10 +866,11 @@ class TrainStep:
     The forward is `forward_train` (the reference's training-mode output dict).  Losses of this benchmark step: L1 rgb, L2 semantics
     (loss_terms.py:14-21, :60-70) and the eikonal term (volsdf_utils.py:19-48; loss.py:83-87); the full reference loss incl. the
     kaolin-target terms (mano_cano, opacity_sparse) is `Loss` (pinned to the reference's module, tests/test_cpu_loss.py) on the
-    same output dict once the canonical meshes are attached to the nodes."""
+    same output dict once the canonical meshes are attached to the nodes.  fused=True: the forward's per-point glue on the fused
+    kernels (forward_train(fused=True))."""
 
-    def __init__(self, net, lr=1e-4, n_eik=256, group=None, capturable=False):
-        self.net, self.group, self.n_eik = net, group, n_eik
+    def __init__(self, net, lr=1e-4, n_eik=256, group=None, capturable=False, fused=False):
+        self.net, self.group, self.n_eik, self.fused = net, group, n_eik, fused
         self.params = [p for p in net.parameters() if p.requires_grad]
         self.opt = torch.optim.Adam(self.params, lr=lr, capturable=capturable)
         self._graph = None
@@ -808,7 +913,7 @@ class TrainStep:
         return self._loss, self._parts
 
     def forward_loss(self, input, gt_rgb, gt_mask, generator=None):
-        out = forward_train(self.net, input, generator)
+        out = forward_train(self.net, input, generator, fused=self.fused)
         B = input["uv"].shape[0]
         eik = [((out[k].norm(2, dim=-1) - 1) ** 2).mean() for k in out if k.endswith("grad_theta")]
         if not eik:   # no canonical meshes attached to the nodes: the global branch (volsdf_utils.py:36-43), uniform in [-0.3, 0.3]^3

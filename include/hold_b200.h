@@ -325,6 +325,41 @@ int hold_forward_warp(hold_ctx* ctx, int node, int B, int P, const float* x_c, c
 int hold_inverse_warp_bwd(hold_ctx* ctx, int node, int B, int P, const float* x, const hold_node_pose* pose, const int32_t* knn_idx,
                           const float* g_xc, float* g_tfs, float* g_x, void* stream);
 
+/* ---- Fused glue of the training forward and its reverse mode (hold_b200/csrc/train_glue.cuh; arithmetic in train_glue_phases.h).
+ * Every stash, scratch and output is caller-allocated (a node's stash must survive until its backward, whatever other nodes run in
+ * between); no call allocates or synchronises the host, so a training step that uses them stays capturable as one CUDA graph.
+ *
+ * hold_train_glue_sizes: floats of the stash hold_normal_density writes for B x P points of `node` (hand 25, object 9 per point)
+ * and of the scratch hold_normal_density_bwd needs (per-block partial sums).  Either pointer may be NULL. */
+int hold_train_glue_sizes(hold_ctx* ctx, int node, int B, int P, int64_t* stash_floats, int64_t* scratch_floats);
+/* extract_features' normal and the Laplace density in training (engine/volsdf_utils.py:66-102, engine/density.py:21-26) for
+ * frame-major points [B,P]: J = (sum_j w_j tfs_j)[:3,:3] with w the detached skinning weights of x_c's 15 nearest CANONICAL
+ * vertices (hand; tfs [B,16,4,4]) or tfs[:3,:3] (object; tfs [B,4,4], x_c unused and may be NULL); g = d sdf / d x_c [B*P,3],
+ * sdf [B*P], beta: device scalar, the effective beta (|beta| + beta_min).  -> normal = normalize(g . J^-1, eps 1e-6) [B*P,3],
+ * density [B*P], stash (hold_train_glue_sizes) for the backward. */
+int hold_normal_density(hold_ctx* ctx, int node, int B, int P, const float* x_c, const float* grad, const float* sdf,
+                        const float* tfs, const float* beta, float* normal, float* density, float* stash, void* stream);
+/* Reverse mode of hold_normal_density from its stash: seeds d_normal [B*P,3] and d_density [B*P] (each may be NULL = 0) ->
+ * d_grad [B*P,3], d_sdf [B*P] (0 where sdf == 0), d_tfs (overwritten; only the 3x3 blocks are non-zero) and d_beta [1].  scratch:
+ * hold_train_glue_sizes.  Fixed-order sums: bitwise reproducible from run to run. */
+int hold_normal_density_bwd(hold_ctx* ctx, int node, int B, int P, const float* grad, const float* sdf, const float* beta,
+                            const float* stash, const float* d_normal, const float* d_density, float* d_grad, float* d_sdf,
+                            float* d_tfs, float* d_beta, float* scratch, void* stream);
+/* The background's network inputs for R rays (background.py:35-100): for the 32 inverse-sphere depths of every ray, emb_pts
+ * [R*32,84] = PE-10 of depth2pts_outside (:102-135) and emb_view [R*32,27] = PE-4 of the ray direction. */
+int hold_bg_inputs(hold_ctx* ctx, int R, float r_sphere, const float* cam_loc, const float* ray_dirs, float* emb_pts,
+                   float* emb_view, void* stream);
+/* bg_volume_rendering of the 32 samples per ray (background.py:137-165) + Background.forward's outputs: sdf at sdf[(r*32+k)*ld_sdf]
+ * (column 0 of the background SDF net's [R*32, 257] output: ld_sdf = 257), rgb [R*32,3], fg_bg_weights [R] -> bg_rgb [R,3],
+ * bg_rgb_only [R,3], bg_semantics [R,4] (each may be NULL). */
+int hold_bg_integrate(hold_ctx* ctx, int R, float r_sphere, const float* sdf, int ld_sdf, const float* rgb, const float* fg_bg_weights,
+                      float* bg_rgb, float* bg_rgb_only, float* bg_semantics, void* stream);
+/* Reverse mode of hold_bg_integrate: seeds of its three outputs (each may be NULL = 0) -> d_rgb [R*32,3], d_sdf [R*32] (contiguous;
+ * 0 where sdf == 0), d_fg_bg_weights [R]. */
+int hold_bg_integrate_bwd(hold_ctx* ctx, int R, float r_sphere, const float* sdf, int ld_sdf, const float* rgb,
+                          const float* fg_bg_weights, const float* g_bg_rgb, const float* g_bg_rgb_only, const float* g_bg_semantics,
+                          float* d_rgb, float* d_sdf, float* d_fg_bg_weights, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
